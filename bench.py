@@ -9,6 +9,7 @@ task prompt / DESIGN.md section "Measurement". Prints ONE JSON line on rank 0.
   python bench.py [--gpus N] [--steps K] [--warmup W]            # B200 arm
   python bench.py --impl reference [--steps K] [--warmup W]      # the reference's own CPU path on the host cores
   python bench.py --config 5                                     # BASELINE.json configs[4]: 736^2 (720 padded), K=512, B=4/GPU
+  python bench.py --dump-outputs DIR                             # also write the last timed step's logits (sample) to DIR
 """
 import argparse
 import json
@@ -27,6 +28,32 @@ sys.path.insert(0, ROOT)
 NET_KW = dict(backbone="clip_vitl16_384", features=256, crop_size=480, arch_option=0, block_depth=0,
               activation="lrelu")
 METRIC = "images/sec at 480x480 ADE20K-150 forward"
+
+
+DUMP_SAMPLE = 1 << 21  # logit values --dump-outputs writes when the step's logits are larger than that
+
+
+def sample_outputs(logits):
+    """The logits of one step as {name: float32/float64 array}: all of them up to DUMP_SAMPLE values, else DUMP_SAMPLE
+    values at flat indices drawn from a fixed seed (the same indices for the same shape in every run, so that two builds
+    can be compared value for value). Runs on the device; only the sample is copied to the host."""
+    import numpy as np
+    flat = logits.detach().reshape(-1)
+    out = {"logits_shape": np.array(logits.shape, dtype=np.float64)}
+    if flat.numel() <= DUMP_SAMPLE:
+        out["logits"] = flat.float().cpu().numpy()
+        return out
+    idx = np.sort(np.random.Generator(np.random.PCG64(0)).integers(0, flat.numel(), size=DUMP_SAMPLE))
+    out["logits"] = flat[torch.from_numpy(idx).to(flat.device)].float().cpu().numpy()
+    out["logits_index"] = idx.astype(np.float64)  # exact: numel < 2**53
+    return out
+
+
+def write_outputs(path, arrays):
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 def ade_labels():
@@ -129,7 +156,7 @@ def cpu_reference_rate(steps, warmup, labels, size):
     """images/sec of the reference's CPU path, one image of the workload per step.
 
     kind "reference": the UNMODIFIED reference `LSegModule.evaluate_random` (modules/lsegmentation_module.py:54-59 ->
-    modules/models/lseg_net.py:160-205) from baseline/_ref (oracle/make_ref.sh), with the stand-ins of
+    modules/models/lseg_net.py:160-205) from the checkout named by LSEG_REFERENCE_ROOT, with the stand-ins of
     oracle/ref_standins.py for the absent third-party packages; kind "port": the oracle restatement when the reference
     tree is not installed. The reference re-runs the text tower on every call (lseg_net.py:183); `text_cached` subtracts
     a separately timed encode_text so that both accountings are visible."""
@@ -178,7 +205,7 @@ def run_reference(args, cfg):
     if rank != 0:
         return
     labels = cfg["labels"]
-    steps = max(1, args.steps)
+    steps = args.steps
     r = cpu_reference_rate(steps, max(1, min(args.warmup, 2)), labels, cfg["size"])
     sample = (f"one {cfg['size']}x{cfg['size']} image of the batch-{cfg['batch']} workload per step (K={len(labels)} labels), "
               f"{steps} steps; the reference re-runs the text tower on every call")
@@ -257,7 +284,13 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-eval", action="store_true", help="skip the multi-scale evaluator line (SURVEY 8(f) row 1)")
     ap.add_argument("--dump-profile", default=None, help="write the per-launch profile of one step to this JSON file")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write the logits of the last timed step (rank 0; a seeded sample, see sample_outputs) as DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes what the B200 arm computes")
     cfg = make_config(args)
     if args.impl == "reference":
         return run_reference(args, cfg)
@@ -308,7 +341,7 @@ def main():
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         return float(t.item())
 
-    W, Ksteps = max(3, args.warmup), max(1, args.steps)
+    W, Ksteps = max(3, args.warmup), args.steps
     out = torch.empty((B, K, S, S), dtype=torch.float32, device=dev)
     for _ in range(W):
         eng.forward(x, text, K, out=out)
@@ -329,6 +362,8 @@ def main():
         ends[i].record()
     barrier()
     t_wall = time.perf_counter() - t_wall0
+    if args.dump_outputs and dist is None:
+        write_outputs(args.dump_outputs, sample_outputs(out))
     clocks = sampler.summary() if world == 1 else None
     compute_ms = max_over_ranks(sum(s.elapsed_time(e) for s, e in zip(starts, ends)))
     compute_value = world * B * Ksteps / (compute_ms / 1e3)
@@ -392,6 +427,8 @@ def main():
         g0.close()
         del g0
         g, full, total_ms, t_wall, clocks = run_gather(True)
+        if args.dump_outputs and rank == 0:
+            write_outputs(args.dump_outputs, sample_outputs(full))
         value = world * B * Ksteps / (total_ms / 1e3)
         wd = ops.read_watchdog()
         check = None

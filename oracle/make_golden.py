@@ -1,6 +1,6 @@
 """TEST INFRASTRUCTURE — generate the golden fixtures under tests/golden/ from the REAL reference.
 
-Runs ONLY in the build container (needs /root/reference): imports the reference's
+Runs only where a lang-seg checkout is named by LSEG_REFERENCE_ROOT: imports the reference's
 modules/models/lseg_net.py unchanged through oracle/ref_standins.py, loads the seeded synthetic state
 dict (oracle/synth.py), runs LSegNet.forward on seeded inputs, verifies that the oracle restatement
 (oracle/lseg_oracle.py) reproduces it, and writes small fixtures:
@@ -13,7 +13,7 @@ dict (oracle/synth.py), runs LSegNet.forward on seeded inputs, verifies that the
   tests/golden/ref_zs.npz       zero-shot path (lseg_net_zs.py) B=3, 96x96, PASCAL label file
   tests/golden/state_dict_keys.json : key -> shape contract of the reference LSegNet
 
-Usage:  python oracle/make_golden.py
+Usage:  LSEG_REFERENCE_ROOT=<lang-seg checkout> python oracle/make_golden.py
 """
 import json
 import os

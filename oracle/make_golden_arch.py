@@ -5,7 +5,7 @@ arch_option 1 (bottleneck_block, block_depth 2, lrelu) and 2 (depthwise_block, b
 state dict (oracle/synth.py, head_block=True), runs it on a seeded input, checks that the oracle restatement
 (oracle/lseg_oracle.py::head_block) reproduces it, and writes tests/golden/ref_arch.npz.
 
-Usage:  python oracle/make_golden_arch.py
+Usage:  LSEG_REFERENCE_ROOT=<lang-seg checkout> python oracle/make_golden_arch.py
 """
 import os
 import sys

@@ -9,7 +9,7 @@ it constructs the unmodified reference LSegNet, loads the seeded state dict (ora
 seeded inputs, checks that the oracle restatement reproduces it (image trunk to 1e-5, logits within the fp16 text-tower
 floor), and writes tests/golden/ref_<tag>.npz and tests/golden/state_dict_keys_<tag>.json (key -> shape contract).
 
-Usage:  python oracle/make_golden_backbones.py [b32] [rn50x16]
+Usage:  LSEG_REFERENCE_ROOT=<lang-seg checkout> python oracle/make_golden_backbones.py [b32] [rn50x16]
 """
 import json
 import os

@@ -6,7 +6,7 @@ small, exactly batch-invariant stand-in network (elementwise arithmetic only), a
 and outputs in tests/golden/ref_multiscale.npz. tests/test_evaluator_cpu.py replays them through
 lseg_b200.evaluator.MultiScaleEvaluator.
 
-    python oracle/make_golden_eval.py        # needs /root/reference (this container only)
+    LSEG_REFERENCE_ROOT=<lang-seg checkout> python oracle/make_golden_eval.py
 """
 import contextlib
 import io
@@ -18,7 +18,6 @@ import torch
 import torch.nn as nn
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
 
 
 class StandInNet(nn.Module):
@@ -49,7 +48,7 @@ CASES = [  # (h, w, base_size, crop_size, scales, K, flip)
 
 
 def main():
-    sys.path.insert(0, REF)
+    sys.path.insert(0, os.environ["LSEG_REFERENCE_ROOT"])
     with contextlib.redirect_stdout(io.StringIO()):
         import additional_utils.models as ref_models
     torch.Tensor.cuda = lambda self, *a, **k: self  # the reference hard-codes .cuda(); we are on CPU

@@ -8,7 +8,7 @@ oracle restatement (oracle/lseg_oracle.py::lseg_forward_rn_zs — torchvision's 
 ResNet stages and path_1 to 1e-5, logits within the fp16 text-tower floor), and writes tests/golden/ref_rn101.npz and
 tests/golden/state_dict_keys_rn101.json.
 
-Usage:  python oracle/make_golden_rn.py
+Usage:  LSEG_REFERENCE_ROOT=<lang-seg checkout> python oracle/make_golden_rn.py
 """
 import json
 import os

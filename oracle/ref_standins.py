@@ -1,4 +1,4 @@
-"""TEST INFRASTRUCTURE — stand-ins that let /root/reference's own modules import and run unchanged.
+"""TEST INFRASTRUCTURE — stand-ins that let the reference's own modules import and run unchanged.
 
 The reference depends on third-party packages that are not installed here (timm 0.4.12, OpenAI clip
 @04f4dc2, PyTorch-Encoding, pytorch_lightning, matplotlib; SURVEY.md Appendix B). This module registers
@@ -9,9 +9,9 @@ The reference depends on third-party packages that are not installed here (timm 
     fp32-computing LayerNorm), weights converted to fp16 like clip.load(device='cuda') does;
     `clip.tokenize` -> oracle.synth.tokenize (no BPE vocabulary offline);
   * inert stubs for encoding / pytorch_lightning / matplotlib so modules/lseg_module.py imports.
-Used by make_golden.py, by the tests that drive the unmodified reference (they skip when neither /root/reference nor
-the baseline/_ref copy made by oracle/make_ref.sh is present) and by bench.py --impl reference; nothing here is
-imported by the product path.
+Used by the fixture generators oracle/make_golden*.py and by bench.py --impl reference (which falls back to the oracle
+restatement when no reference checkout is given); nothing here is imported by the product path. The checkout is named
+by the environment variable LSEG_REFERENCE_ROOT.
 """
 import os
 import sys
@@ -21,22 +21,11 @@ from collections import OrderedDict
 import torch
 import torch.nn as nn
 
-def _find_reference_root():
-    """/root/reference in the build container; on the GPU box the byte-for-byte copy oracle/make_ref.sh installs under
-    baseline/_ref/ (git-ignored, travels with the gpurun snapshot)."""
-    here = os.path.dirname(os.path.abspath(__file__))
-    for cand in (os.environ.get("LSEG_REFERENCE_ROOT"), "/root/reference",
-                 os.path.join(os.path.dirname(here), "baseline", "_ref")):
-        if cand and os.path.isdir(os.path.join(cand, "modules", "models")):
-            return cand
-    return "/root/reference"
-
-
-REFERENCE_ROOT = _find_reference_root()
+REFERENCE_ROOT = os.environ.get("LSEG_REFERENCE_ROOT", "")  # a lang-seg checkout
 
 
 def reference_available():
-    return os.path.isdir(os.path.join(REFERENCE_ROOT, "modules", "models"))
+    return bool(REFERENCE_ROOT) and os.path.isdir(os.path.join(REFERENCE_ROOT, "modules", "models"))
 
 
 # ---------------------------------------------------------------------------------------------
@@ -224,9 +213,9 @@ def _clip_load(name, device="cpu", jit=False):
 
 
 def install(with_lightning_stack=True):
-    """Register the stand-ins and put /root/reference on sys.path. Idempotent."""
+    """Register the stand-ins and put the reference checkout on sys.path. Idempotent."""
     if not reference_available():
-        raise FileNotFoundError(f"{REFERENCE_ROOT} is not available (run oracle/make_ref.sh in the build container)")
+        raise FileNotFoundError(f"no lang-seg checkout at LSEG_REFERENCE_ROOT={REFERENCE_ROOT!r}")
     here = os.path.dirname(os.path.abspath(__file__))
     sys.path.insert(0, os.path.dirname(here))
     from oracle import synth

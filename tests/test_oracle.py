@@ -2,7 +2,7 @@
   * against the golden fixtures generated from the REAL reference (oracle/make_golden.py);
   * the restated third-party blocks (timm ViT block, CLIP text tower) against transformers' independent
     implementations with shared random weights (SURVEY.md section 8(c) item 2);
-  * when /root/reference is present (build container only): a live re-run of the reference's own files.
+  * a small forward of the reference's own files, recorded as a fixture (oracle/make_golden_callers.py).
 """
 import json
 import os
@@ -20,6 +20,16 @@ torch.set_num_threads(max(1, min(16, os.cpu_count() or 1)))
 # order only; measured 2.0e-3 of max|logit| when the fixtures were generated (make_golden.py log).
 TEXT_FP16_TOL = 3e-3
 
+# The image trunk is restated op for op: bit-identical to the fixtures on the CPU they were recorded on. Another x86
+# vector ISA (the AVX2 / SSE4 kernels of MKL, oneDNN and ATen) sums fp32 in another order: measured 1.1e-6 of max|t| on
+# a trunk row and 8e-6 on a tensor mean. TRUNK_REL bounds the former, TRUNK_STATS_RTOL the latter.
+TRUNK_REL = 1e-5
+TRUNK_STATS_RTOL = 5e-5
+
+
+def assert_trunk_row(got, want):
+    assert rel_err(got, torch.from_numpy(want)) <= TRUNK_REL, rel_err(got, torch.from_numpy(want))
+
 
 def test_small_golden_matches_oracle():
     z = np.load(os.path.join(GOLD, "ref_small.npz"))
@@ -29,12 +39,12 @@ def test_small_golden_matches_oracle():
     ref = torch.from_numpy(z["logits"])
     assert out.shape == ref.shape == (2, 5, 64, 96)
     assert rel_err(out, ref) < TEXT_FP16_TOL
-    # the image trunk is restated op for op -> bit-identical intermediate tensors
-    assert torch.equal(st["taps"][3][0, 0], torch.from_numpy(z["tap3_row0"]))
+    # the image trunk is restated op for op -> identical intermediate tensors up to the CPU's fp32 summation order
+    assert_trunk_row(st["taps"][3][0, 0], z["tap3_row0"])
     for i in range(4):
         t = st["taps"][i]
         got = np.array([t.mean().item(), t.std().item(), t.abs().max().item()])
-        assert np.allclose(got, z["taps_stats"][i], rtol=1e-6, atol=1e-7)
+        assert np.allclose(got, z["taps_stats"][i], rtol=TRUNK_STATS_RTOL, atol=1e-7)
 
 
 @pytest.mark.parametrize("tag,labels", [("k2", ["cat", "other"]), ("k150", None)])
@@ -46,7 +56,7 @@ def test_480_golden_matches_oracle(tag, labels):
     out, st = O.lseg_forward(x, synth.tokenize(labels), state_dict(0), return_stages=True)
     lat = torch.from_numpy(z["logits_lattice"])
     assert rel_err(out[:, :, ::8, ::8], lat) < TEXT_FP16_TOL
-    assert torch.equal(st["taps"][3][0, 0], torch.from_numpy(z["tap3_row0"]))
+    assert_trunk_row(st["taps"][3][0, 0], z["tap3_row0"])
     tf = torch.from_numpy(z["text_features"]).float()
     cos = torch.nn.functional.cosine_similarity(st["text_features"].float(), tf, dim=-1)
     assert cos.min() > 0.9999
@@ -220,7 +230,7 @@ def test_reference_key_contract():
     ("rn50x16", "clipRN50x16_vitl16_384", [(256, 16, 24), (512, 8, 12), (1024, 4, 6), (1024, 2, 3)])])
 def test_other_backbone_golden_and_key_contract(tag, backbone, layer_shapes):
     """The oracle against the unmodified reference's output with that backbone (oracle/make_golden_backbones.py), trunk
-    statistics to 1e-6, and the drop-in module's state-dict keys/shapes against the reference module's."""
+    statistics to the CPU's fp32 summation order (TRUNK_STATS_RTOL), and the drop-in module's state-dict keys/shapes against the reference module's."""
     import lseg_b200  # noqa: F401
     from lseg_b200.lseg_net import LSegNet
     from parity_util import NET_KW
@@ -232,11 +242,11 @@ def test_other_backbone_golden_and_key_contract(tag, backbone, layer_shapes):
     ref = torch.from_numpy(z["small_logits"])
     assert out.shape == ref.shape == (2, 5, 64, 96)
     assert rel_err(out, ref) < 5e-3  # two executions of the fp16 text tower (measured 3.0e-3 at max|logit| ~ 0.3)
-    assert torch.equal(st["taps"][3][0, 0], torch.from_numpy(z["small_tap3_row0"]))
+    assert_trunk_row(st["taps"][3][0, 0], z["small_tap3_row0"])
     for i in range(4):
         for name, t in (("taps", st["taps"][i]), ("layers", st["layers"][i])):
             got = np.array([t.mean().item(), t.std().item(), t.abs().max().item()])
-            assert np.allclose(got, z[f"small_{name}_stats"][i], rtol=1e-6, atol=1e-7), (name, i)
+            assert np.allclose(got, z[f"small_{name}_stats"][i], rtol=TRUNK_STATS_RTOL, atol=1e-7), (name, i)
     assert [tuple(l.shape[1:]) for l in st["layers"]] == layer_shapes
     want = json.load(open(os.path.join(GOLD, f"state_dict_keys_{tag}.json")))
     net = LSegNet(labels=["a", "b"], **{**NET_KW, "backbone": backbone})
@@ -249,7 +259,7 @@ def test_other_backbone_golden_and_key_contract(tag, backbone, layer_shapes):
 
 def test_rn101_zero_shot_golden_and_key_contract():
     """LSegRNNetZS (ResNet-101 trunk, lseg_net_zs.py:240-378): the oracle against the unmodified reference's output
-    (oracle/make_golden_rn.py), stage statistics to 1e-6, and the drop-in module's state-dict keys/shapes."""
+    (oracle/make_golden_rn.py), stage statistics to TRUNK_STATS_RTOL, and the drop-in module's state-dict keys/shapes."""
     import lseg_b200  # noqa: F401
     from lseg_b200.lseg_net import LSegNetZS, LSegRNNetZS
     z = np.load(os.path.join(GOLD, "ref_rn101.npz"))
@@ -265,7 +275,7 @@ def test_rn101_zero_shot_golden_and_key_contract():
     for k in range(4):
         t = st["layers"][k]
         got = np.array([t.mean().item(), t.std().item(), t.abs().max().item()])
-        assert np.allclose(got, z["small_layers_stats"][k], rtol=1e-6, atol=1e-7), k
+        assert np.allclose(got, z["small_layers_stats"][k], rtol=TRUNK_STATS_RTOL, atol=1e-7), k
     want = json.load(open(os.path.join(GOLD, "state_dict_keys_rn101.json")))
     net = LSegRNNetZS(label_list=names, features=256, arch_option=0, block_depth=0, activation="lrelu")
     assert {k: list(v.shape) for k, v in net.state_dict().items()} == want
@@ -314,13 +324,12 @@ def test_tokenizer_contract():
         tokenize(["w " * 100])
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference"), reason="reference tree only exists in the build container")
 def test_live_reference_small():
-    from oracle import ref_standins as R
-    labels = ["cat", "other", "tree"]
-    net = R.build_reference_net(state_dict(0), labels)
-    x = synth.make_image(1, 64, 64, seed=9)
-    with torch.no_grad():
-        ref = net(x)
+    """The unmodified reference LSegNet.forward on one 64x64 image, as recorded by oracle/make_golden_callers.py."""
+    z = np.load(os.path.join(GOLD, "ref_live_small.npz"))
+    labels = [str(s) for s in z["labels"]]
+    x = synth.make_image(*[int(v) for v in z["shape"][[0, 2, 3]]], seed=int(z["seed"]))
+    ref = torch.from_numpy(z["logits"])
     got = O.lseg_forward(x, synth.tokenize(labels), state_dict(0))
+    assert got.shape == ref.shape == (1, 3, 64, 64)
     assert rel_err(got, ref) < TEXT_FP16_TOL
